@@ -24,6 +24,9 @@ the rank that writes the matrix (`--gather root`, ncclSend/Recv) and overlapped 
            the timed steps; `roofline.issue_bound` is the same kernel against the ALU-pipe bound that actually binds.
 `cpu_baseline`: the oracle's C port of the reference algorithm timed on this box's host cores (bounded sample), with its
            thread scaling and the cgroup CPU quota, so that a CPU-starved box explains itself.
+
+`--dump-outputs DIR` writes the triplets the last timed `value` step returned as float64 .npy files (see dump_outputs),
+so that two builds run with the same arguments -- hence the same seeded shard -- can be compared output for output.
 """
 from __future__ import annotations
 
@@ -44,10 +47,17 @@ METRIC = "reads_sw_scored_per_sec"
 UNIT = "pairs/s"
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
+
+
 def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5, help="timed steps of each measured path")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="vartrix_b200", choices=["vartrix_b200", "reference"])
     ap.add_argument("--workload", default="config3", help="synth.CONFIGS key (config3 = the shape the metric is quoted on)")
@@ -62,6 +72,7 @@ def parse_args(argv=None):
     ap.add_argument("--growth", type=float, default=2.0, help="e2e shards grow geometrically from --first-chunk by this factor (0: equal shards after the first)")
     ap.add_argument("--first-chunk", type=float, default=0.01, help="fraction of the candidates in the first (priming) shard")
     ap.add_argument("--min-shard", type=int, default=100_000, help="e2e shards are not made smaller than this many candidates (per-submit fixed costs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="write the last timed step's triplets to DIR/<name>.npy (one process only)")
     return ap.parse_args(argv)
 
 
@@ -289,6 +300,24 @@ def triplet_checksum(row, col, val):
         return int(x.sum(dtype=np.uint64))
 
 
+DUMP_MAX_ENTRIES = 1 << 20      # 4 float64 arrays of 1 M entries = 32 MB
+
+
+def dump_outputs(out_dir, res, with_val2):
+    """Write `res` (Triplets) to out_dir as float64 .npy files: row, col, val and, when the mode fills a ref matrix, val2,
+    each at the same positions -- all of them, or a seeded sample of DUMP_MAX_ENTRIES in triplet order when there are
+    more -- plus metrics.npy = [triplets, num_scored, num_not_cell_bc, num_non_umi] of the whole result."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(res.row)
+    idx = np.arange(n)
+    if n > DUMP_MAX_ENTRIES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENTRIES, replace=False))
+    for name in ("row", "col", "val") + (("val2",) if with_val2 else ()):
+        np.save(os.path.join(out_dir, f"{name}.npy"), getattr(res, name)[idx].astype(np.float64))
+    m = res.metrics
+    np.save(os.path.join(out_dir, "metrics.npy"), np.array([n, m["num_scored"], m["num_not_cell_bc"], m["num_non_umi"]], np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
@@ -301,6 +330,8 @@ def run_gpu(args):
     rank, world, local = dist_env()
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: vartrix_b200 has no CPU fallback (use --impl reference for the CPU arm)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the result of one process: run it without torchrun")
     # stdout carries exactly one JSON line: anything native libraries print there (e.g. NCCL's version banner)
     # goes to stderr instead
     sys.stdout.flush()
@@ -454,6 +485,8 @@ def run_gpu(args):
     gather_flush()
     sampler = ClockSampler(local) if rank == 0 else None
     ms, sw_ms, launches, last, clocks = timed(step_device, args.steps, sampler)
+    if args.dump_outputs:       # before the e2e steps below reuse the engine's result arrays
+        dump_outputs(args.dump_outputs, eng.fetch(last), cfg["scoring_method"] == "coverage")
     total_pairs = n_pairs * world
     if world > 1:
         tp = torch.tensor([n_pairs], device="cuda", dtype=torch.int64); dist.all_reduce(tp); total_pairs = int(tp.item())
@@ -591,6 +624,8 @@ def run_gpu(args):
 def main():
     args = parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes what the CUDA path computed (--impl vartrix_b200)")
         return run_reference(args)
     return run_gpu(args)
 

@@ -5,12 +5,15 @@ oracle.pipeline (Python decode + C oracle) and compares every output with the co
 golden `.mtx` as a (row, col) -> value set, exactly like the reference's
 `assert_eq!(seen.to_csr(), expected.to_csr())` (main.rs:1230-1232).
 
-Usage:  python -m oracle.check_goldens [reference_test_dir]      (default /root/reference/test)
+Usage:  python -m oracle.check_goldens [reference_test_dir]      (default tests/golden/ref_inputs)
 """
 import math
+import os
 import sys
 
 from . import pipeline as P
+
+REF_TEST_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "ref_inputs")
 
 CASES = [  # (name, main.rs lines, files prefix, barcodes, mode, umi, golden out, golden ref)
     ("test_consensus_matrix", "1207-1233", "test", "barcodes.tsv", "consensus", False, "test_consensus.mtx", None),
@@ -36,7 +39,7 @@ def same(a, b):
     return all((math.isnan(a[k]) and math.isnan(b[k])) or a[k] == b[k] for k in a)
 
 
-def main(test_dir="/root/reference/test"):
+def main(test_dir=REF_TEST_DIR):
     ok = True
     for name, lines, pre, bcs, mode, umi, g_out, g_ref in CASES:
         nr, nc, res, batch, _ = P.run_files(f"{test_dir}/{pre}.vcf", f"{test_dir}/{pre}.bam", f"{test_dir}/{pre}.fa",

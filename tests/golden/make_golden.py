@@ -1,7 +1,7 @@
-"""Regenerates tests/golden/*.npz|json from the reference's own fixtures (run in the build container,
-where /root/reference exists; the GPU box only sees the committed outputs).
+"""Regenerates tests/golden/*.npz|json from the reference's own fixtures (by default the verbatim copy of the
+reference's test/ directory in tests/golden/ref_inputs).
 
-  python tests/golden/make_golden.py [/root/reference/test]
+  python tests/golden/make_golden.py [reference_test_dir]
 
 Outputs
   rna_batch.npz / dna_batch.npz : the staged candidates of test/test.{vcf,bam,fa} and test/test_dna.*
@@ -21,7 +21,7 @@ from oracle.check_goldens import CASES    # noqa: E402
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def main(test_dir="/root/reference/test"):
+def main(test_dir=os.path.join(HERE, "ref_inputs")):
     for pre, out in (("test", "rna_batch.npz"), ("test_dna", "dna_batch.npz")):
         b = P.stage_from_files(f"{test_dir}/{pre}.vcf", f"{test_dir}/{pre}.bam", f"{test_dir}/{pre}.fa")
         b.save(os.path.join(HERE, out))

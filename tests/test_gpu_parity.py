@@ -294,6 +294,26 @@ def test_device_resident_submit_equals_host_submit(vb):
                 assert got.metrics == exp.metrics
 
 
+def test_bench_dump_outputs_are_the_oracle_triplets(vb, oracle, tmp_path):
+    """bench.py --dump-outputs writes what its timed `value` steps returned: the oracle's triplets of the same seeded shard."""
+    import json
+    import subprocess
+    import sys
+    from conftest import ROOT
+    from vartrix_b200 import dist as vdist
+    d = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "config2", "--loci", "400", "--steps", "2",
+                        "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    sb, bcs, _ = vb.synth.make_shard(**vdist.rank_workload(dict(vb.synth.CONFIGS["config2"], n_loci=400), 0))
+    exp = _oracle_run(oracle, sb, bcs, "coverage", False)
+    for f in ("row", "col", "val", "val2"):
+        assert np.array_equal(np.load(d / f"{f}.npy"), getattr(exp, f).astype(np.float64), equal_nan=True), f
+    m = exp.metrics
+    assert np.array_equal(np.load(d / "metrics.npy"), [len(exp.row), m["num_scored"], m["num_not_cell_bc"], m["num_non_umi"]])
+
+
 def test_edge_cases(vb, oracle):
     sb, bcs, info = vb.synth.make_shard(40, 10, depth=30, seed=3, umi=True, unlisted_frac=0.3)
     # reads without CB / without UB, loci without candidates

@@ -205,3 +205,37 @@ def test_bench_arguments_and_shard_growth_policy():
     assert mod.pick_growth(16.6, 35.3, 1.4) == 1.4            # one GPU: copies are twice as fast as the kernels
     assert 1.15 < mod.pick_growth(27.0, 36.6, 1.4) < 1.3      # eight ranks sharing the host's PCIe paths
     assert mod.pick_growth(80.0, 36.0, 1.4) == 1.1 and mod.pick_growth(0.0, 1.0, 1.4) == 1.4
+    assert mod.parse_args(["--steps", "7"]).steps == 7
+    with pytest.raises(SystemExit):
+        mod.parse_args(["--steps", "0"])
+
+
+def test_bench_dump_outputs_is_a_fixed_capped_sample(tmp_path):
+    """bench.py --dump-outputs: float64 arrays of whole triplets at the same seeded positions every run, 64 MB at most."""
+    import importlib.util
+    import vartrix_b200 as vb
+    spec = importlib.util.spec_from_file_location("vtx_bench", os.path.join(ROOT, "bench.py"))
+    mod = importlib.util.module_from_spec(spec); spec.loader.exec_module(mod)
+    rng = np.random.default_rng(1)
+    n = mod.DUMP_MAX_ENTRIES + 12345
+    row = np.sort(rng.integers(0, 1 << 31, n)).astype(np.uint32)
+    col = rng.integers(0, 1 << 31, n).astype(np.uint32)
+    none = np.zeros(0, np.uint32)
+    res = vb.Triplets(row, col, none, none, none, row * 0.5 + col, -1.0 * col, dict(num_scored=7, num_not_cell_bc=8, num_non_umi=9))
+    for d in ("a", "b"):
+        mod.dump_outputs(str(tmp_path / d), res, True)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["col.npy", "metrics.npy", "row.npy", "val.npy", "val2.npy"]
+    got = {}
+    for nm in names:
+        a, b = np.load(tmp_path / "a" / nm), np.load(tmp_path / "b" / nm)
+        assert a.dtype == np.float64 and np.array_equal(a, b), nm
+        got[nm[:-4]] = a
+    assert sum(os.path.getsize(tmp_path / "a" / nm) for nm in names) <= 64 << 20
+    assert len(got["row"]) == mod.DUMP_MAX_ENTRIES and (np.diff(got["row"]) >= 0).all()        # sampled in triplet order
+    assert np.array_equal(got["val"], got["row"] * 0.5 + got["col"]) and np.array_equal(got["val2"], -got["col"])
+    assert np.array_equal(got["metrics"], [n, 7, 8, 9])
+    small = vb.Triplets(row[:10], col[:10], none, none, none, res.val[:10], none.astype(np.float64), res.metrics)
+    mod.dump_outputs(str(tmp_path / "small"), small, False)
+    assert sorted(os.listdir(tmp_path / "small")) == ["col.npy", "metrics.npy", "row.npy", "val.npy"]
+    assert np.array_equal(np.load(tmp_path / "small" / "row.npy"), row[:10])
