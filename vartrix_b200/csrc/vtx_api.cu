@@ -261,13 +261,22 @@ int launch_sw_split(vtx_ctx* ctx, SwArgs a, uint64_t* launches)
 
 int launch_sw_fold(vtx_ctx* ctx, SwArgs a, uint64_t* launches)
 {
-    const size_t smem = fold_warp_bytes() * (kFoldThreads / 32);
+    // The allele table holds the widest window's allele columns: max_hap_len is exact for host batches and, for device
+    // batches, a promise that vtx_k_locus_prep enforces (a wider locus gets no tiles).
+    a.fold_mid_cap = std::min(std::max(int(a.max_hap) - 2 * kFoldP, 1), kFoldMaxMid);
+    const size_t wb = fold_warp_bytes(a.fold_mid_cap);
     auto kern = vtx_k_sw_fold;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kFoldThreads, smem));
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(wb * (kFoldThreads / 32))));
+    // 9 warps per CTA when two such CTAs fit an SM (SNV windows), otherwise 8 (wide indel windows)
+    int threads = kFoldThreads, per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, wb * (threads / 32)));
+    if (per_sm < 2) {
+        threads = kFoldThreadsNarrow;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, wb * (threads / 32)));
+    }
+    const size_t smem = wb * (threads / 32);
     if (per_sm < 1) return set_err(ctx, VTX_E_CUDA, "folded SW kernel does not fit on an SM (smem %zu)", smem);
-    kern<<<ctx->n_sm * per_sm, kFoldThreads, smem, ctx->stream>>>(a);
+    kern<<<ctx->n_sm * per_sm, threads, smem, ctx->stream>>>(a);
     CK(cudaGetLastError());
     ++*launches;
     return VTX_OK;

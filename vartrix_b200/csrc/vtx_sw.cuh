@@ -140,6 +140,7 @@ struct SwArgs {
     uint32_t k64k;                  // 65536 as a run-time value (keeps a shift-add on the FMA pipe, see vtx_sw_split.cuh)
     uint32_t one;                   // 1 as a run-time value (keeps the packed adds on the FMA pipe)
     int32_t multi;                  // class 3 may run several column passes (boundary buffer present in smem)
+    int32_t fold_mid_cap;           // folded kernel: allele columns its per-warp table holds (set by launch_sw_fold)
     // generic kernel only
     uint32_t* scratch;              // [warps][max_hap + 1][32]
     uint32_t max_hap;

@@ -15,9 +15,10 @@
 //
 //   main pass   kFoldP = 96 columns, 12 per lane, rows skewed by one step per lane exactly like the other
 //               kernels -- but the two int16 halves are (forward DP over hap[0, 96), reversed DP over
-//               hap[n - 96, n) reversed) of the SAME read.  Per step a lane fetches the forward and the reverse
-//               profile row (LDS.128) and merges them with an IMAD.  The last column (H + gap, E) of every
-//               row goes to shared memory.
+//               hap[n - 96, n) reversed) of the SAME read.  Row i of the read meets forward code f = read[i] and reverse
+//               code r = read[m - 1 - i], so the profile is pre-merged over the 16 (f, r) pairs of ACGT plus one
+//               all-mismatch row: per step a lane loads one code byte (4 f + r) and one profile row (3 LDS.128), used as
+//               loaded.  The last column (H + gap, E) of every row goes to shared memory.
 //   middle      the n - 192 allele columns (9 for an SNV with --padding 100, up to 40): halves are (ref, alt)
 //               again.  Transposed wavefront: lane g owns the 19 read rows [19 g, 19 g + 19), whose (H + gap, E)
 //               start from the parked forward boundary, and walks over the columns one step per column,
@@ -28,6 +29,11 @@
 // Per pair this is 2 x 96 + (n - 192) column-passes in "one read per word" units instead of 96 / 2 + (n - 96):
 // ~25 % fewer DPX instructions than vtx_k_sw_split for an SNV window.  Reads up to kFoldMaxRead bases,
 // windows with both flanks >= 96 columns in common and at most kFoldMaxMid allele columns.
+//
+// A tile in which some read has a base other than ACGT (N, IUPAC: nib_code 4, matches nothing) has no pair row for
+// it; such tiles (rare: real reads seldom carry an N) run a second instantiation of the main pass whose code byte
+// keeps both codes, f << 3 | r, and which assembles each word from the forward half of row 4 f and the reverse half
+// of row r, taking the all-mismatch row for a code of 4.
 #pragma once
 #include "vtx_sw.cuh"
 
@@ -39,37 +45,35 @@ constexpr int kFoldPPW = 4;            // pairs per warp tile
 constexpr int kFoldR = 19;             // read rows per lane in the middle (8 x 19 = 152)
 constexpr int kFoldMaxRead = 8 * kFoldR;
 constexpr int kFoldMaxMid = 40;        // allele columns: n <= 2 * 96 + 40 = 232
+constexpr int kFoldProfRows = 17;      // pre-merged profile: row 4 f + r for f, r in ACGT, row 16 all mismatch
+constexpr uint8_t kFoldSentinel = 16;            // code byte of a row outside the read
+constexpr uint8_t kFoldSentinelMixed = 4 << 3 | 4;   // the same in the code of the mixed main pass (f << 3 | r)
 // boundary rows kept per read; 156 (not 152) so that the four reads of a tile start 8, 16 and 24 banks apart
 // (152 rows x 8 bytes put reads 0/2 and 1/3 on the same banks: a 2-way conflict on every boundary store and load)
 constexpr int kFoldRows = kFoldMaxRead + 4;
-constexpr int kFoldCodeStride = kFoldMaxRead + 16;   // row codes per read and direction (8 sentinels either side)
-// 288 threads x 2 CTAs = 18 warps/SM at 96 registers (a few spills in the tile prologue only).  Round 1 (unfused cell, no
-// unrolling): 320 x 2 beat 256 x 2 by 5 %; with the fused cell and the row loop unrolled twice 288 x 2 is the best of
-// 256 / 288 / 320 by ~1 % (profiles/r02_fold_variants.txt): the kernel is bound by issue slots and the ALU pipe, not by latency.
+constexpr int kFoldCodeStride = kFoldMaxRead + 16;   // row codes per read (8 sentinels either side)
+// 288 threads x 2 CTAs = 18 warps/SM at 96 registers.  Round 1 (unfused cell, no unrolling): 320 x 2 beat 256 x 2 by 5 %;
+// with the fused cell and the row loop unrolled twice 288 x 2 is the best of 256 / 288 / 320 by ~1 %
+// (profiles/r02_fold_variants.txt): the kernel is bound by issue slots and the ALU pipe, not by latency.  The launch drops to
+// kFoldThreadsNarrow when two 288-thread CTAs do not fit an SM with the allele table the batch needs (wide indel windows).
 #ifndef VTX_FOLD_UNROLL
 #define VTX_FOLD_UNROLL 2
 #endif
-// 1: the reverse profile is stored in the HIGH half, so the (forward | reverse) substitution word is a plain add of the two
-// profile words (eligible for IMAD.IADD / VIADD) instead of a full IMAD b * 65536 + a (half-rate FMA-heavy pipe)
-#ifndef VTX_FOLD_PRESHIFT
-#define VTX_FOLD_PRESHIFT 0
-#endif
-#ifndef VTX_FOLD_THREADS
-#define VTX_FOLD_THREADS 288
-#endif
-constexpr int kFoldThreads = VTX_FOLD_THREADS;
+constexpr int kFoldThreads = 288;
+constexpr int kFoldThreadsNarrow = 256;
 constexpr int kFoldUnroll = VTX_FOLD_UNROLL;         // row-loop unrolling of the main pass
 #ifndef VTX_FOLD_MID_UNROLL
 #define VTX_FOLD_MID_UNROLL 1
 #endif
 constexpr int kFoldMidUnroll = VTX_FOLD_MID_UNROLL;  // column-loop unrolling of the allele pass
 
-__host__ __device__ constexpr size_t fold_warp_bytes()
+// shared memory per warp for allele tables of mid_cap columns (SwArgs::fold_mid_cap, sized at launch from max_hap_len)
+__host__ __device__ inline size_t fold_warp_bytes(int mid_cap)
 {
-    size_t b = size_t(2 * 5 * kFoldP) * 4;                       // forward + reverse profile
-    b += size_t(kFoldMaxMid) * 8 * 4;                            // allele-column table [column][read code]
+    size_t b = size_t(kFoldProfRows * kFoldP) * 4;               // pre-merged (forward | reverse) profile
+    b += size_t(mid_cap) * 8 * 4;                                // allele-column table [column][read code]
     b += size_t(kFoldPPW) * kFoldRows * 8 + 32;                  // boundary column (forward | reverse), per read and row
-    b += size_t(2 * kFoldPPW) * kFoldCodeStride;                 // row codes, forward and reversed
+    b += size_t(kFoldPPW) * kFoldCodeStride;                     // row codes, one byte per row
     return (b + 15) & ~size_t(15);
 }
 
@@ -79,25 +83,94 @@ constexpr int kJuncH = -2 * kGoe - kBias, kJuncE = -kGapOpen - kBias;
 constexpr uint32_t kJuncH2 = (uint32_t(uint16_t(int16_t(kJuncH - 1))) << 16) | uint32_t(uint16_t(int16_t(kJuncH)));
 constexpr uint32_t kJuncE2 = (uint32_t(uint16_t(int16_t(kJuncE - 1))) << 16) | uint32_t(uint16_t(int16_t(kJuncE)));
 
+// low half of a, high half of b: one LOP3 (a & 0xFFFF | b & ~0xFFFF)
+__device__ __forceinline__ uint32_t lop_lo_hi(uint32_t a, uint32_t b)
+{
+    uint32_t d;
+    asm("lop3.b32 %0, %1, %2, %3, 0xE2;" : "=r"(d) : "r"(a), "r"(0x0000FFFFu), "r"(b));
+    return d;
+}
+
+// Main pass of one tile: forward DP over hap[0, P) in the low half, reversed DP over hap[n - P, n) in the high half.
+// Returns the running maximum of the unit (not yet reduced over its lanes); parks (H + gap, E) of column P - 1 / n - P.
+//   MIXED = false: cA[t] is the profile row (4 f + r, kFoldSentinel outside the read).
+//   MIXED = true:  cA[t] = f << 3 | r; the forward half comes from row 4 f (16 for f = 4), the reverse half from row r
+//                  (16 for r = 4).
+template <bool MIXED>
+__device__ __forceinline__ uint32_t fold_main_pass(const uint32_t* __restrict__ prof, const uint8_t* __restrict__ cA, int steps,
+                                                   int g, uint32_t one, uint2* __restrict__ my_bnd)
+{
+    constexpr int C1 = kFoldC1, RS1 = kFoldP;
+    uint32_t hg[C1], f[C1];
+#pragma unroll
+    for (int c = 0; c < C1; ++c) { hg[c] = kGOE2; f[c] = kNEG2; }
+    uint32_t hg_last = kGOE2, e_last = kNEG2, diag_save = kGOE2;
+    uint32_t best = kBIAS2;
+    const uint32_t* lane_p = prof + g * C1;
+#pragma unroll kFoldUnroll
+    for (int t = 0; t < steps; ++t) {
+        uint32_t hl = __shfl_up_sync(0xffffffffu, hg_last, 1, 8);
+        uint32_t el = __shfl_up_sync(0xffffffffu, e_last, 1, 8);
+        if (g == 0) { hl = kGOE2; el = kNEG2; }
+        const uint32_t code = cA[t];
+        const uint4* pa = reinterpret_cast<const uint4*>(lane_p + (MIXED ? (code >> 3) * 4 : code) * RS1);
+        const uint4* pb = reinterpret_cast<const uint4*>(lane_p + ((code & 7) + 3 * (code & 4)) * RS1);   // MIXED only
+        uint32_t diag = diag_save;
+        diag_save = hl;
+        uint32_t e = el, eg = hl, hleft = hl;
+#pragma unroll
+        for (int q = 0; q < C1 / 4; ++q) {
+            uint32_t sv[4];
+            const uint4 a4 = pa[q];
+            if (MIXED) {
+                const uint4 b4 = pb[q];
+                sv[0] = lop_lo_hi(a4.x, b4.x); sv[1] = lop_lo_hi(a4.y, b4.y);
+                sv[2] = lop_lo_hi(a4.z, b4.z); sv[3] = lop_lo_hi(a4.w, b4.w);
+            } else {
+                sv[0] = a4.x; sv[1] = a4.y; sv[2] = a4.z; sv[3] = a4.w;
+            }
+            uint32_t hh[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int c = 4 * q + k;
+                const uint32_t fc = __viaddmax_s16x2(f[c], kGE2, hg[c]);
+                e = __viaddmax_s16x2(e, kGE2, eg);
+                const uint32_t h = sw_h(diag, one, sv[k], fc, e);
+                hh[k] = h;
+                diag = hg[c];
+                hleft = hadd(h, one, c);
+                eg = hleft;
+                hg[c] = hleft;
+                f[c] = fc;
+            }
+            best = __vimax3_s16x2(best, hh[0], hh[1]);
+            best = __vimax3_s16x2(best, hh[2], hh[3]);
+        }
+        hg_last = hleft;
+        e_last = e;
+        if (g == 7) my_bnd[t] = make_uint2(hleft, e);                    // columns P-1 (fwd) / n-P (rev) of row t-7
+    }
+    return best;
+}
+
 __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
 {
-    constexpr int C1 = kFoldC1, P = kFoldP, R = kFoldR, M = 8;
+    constexpr int P = kFoldP, R = kFoldR, M = 8;
     constexpr int RS1 = P;                                       // 96 words: rows stay on their banks
 
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int u = lane >> 3, g = lane & 7;                       // unit = read of the tile, lane within the unit
-    uint8_t* wbase = smem_raw + warp * fold_warp_bytes();
-    uint32_t* profF = reinterpret_cast<uint32_t*>(wbase);
-    uint32_t* profR = profF + 5 * RS1;
-    uint32_t* midtab = profR + 5 * RS1;
-    uint2* bnd = reinterpret_cast<uint2*>(midtab + kFoldMaxMid * 8);
+    const int mid_cap = a.fold_mid_cap;                          // allele columns of the widest window of the batch
+    uint8_t* wbase = smem_raw + warp * fold_warp_bytes(mid_cap);
+    uint32_t* prof = reinterpret_cast<uint32_t*>(wbase);         // [kFoldProfRows][RS1]
+    uint32_t* midtab = prof + kFoldProfRows * RS1;               // [mid_cap][8]
+    uint2* bnd = reinterpret_cast<uint2*>(midtab + mid_cap * 8);
     uint8_t* codes = reinterpret_cast<uint8_t*>(bnd + kFoldPPW * kFoldRows + 4);
 
     const uint32_t n_tiles = __ldg(a.tile_start + a.n_loci);
     uint32_t cached_locus = 0xFFFFFFFFu;
     const uint32_t tile_chunk = max(1u, min(uint32_t(kTileChunk), n_tiles / (gridDim.x * (blockDim.x >> 5) * 16u)));
-    const uint32_t k64k = a.k64k;                                // 65536, opaque to ptxas so the merge stays an IMAD
     const uint32_t one = a.one;
     int mid_ref = 0, mid_alt = 0;                                // allele columns of the cached locus
 
@@ -126,11 +199,11 @@ __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
                     const uint32_t fb = hap_code(__ldg(rh + j));
                     const uint32_t sb = hap_code(__ldg(rh + (n_ref - 1 - j)));
 #pragma unroll
-                    for (uint32_t r = 0; r < 5; ++r) {
-                        profF[r * RS1 + j] = uint32_t(r == fb ? kProfMatch : kProfMis);      // low half only: merged per step
-                        profR[r * RS1 + j] = uint32_t(r == sb ? kProfMatch : kProfMis) << (VTX_FOLD_PRESHIFT ? 16 : 0);
-                    }
+                    for (uint32_t p = 0; p < 16; ++p)
+                        prof[p * RS1 + j] = pack2((p >> 2) == fb ? kProfMatch : kProfMis, (p & 3) == sb ? kProfMatch : kProfMis);
+                    prof[16 * RS1 + j] = pack2(kProfMis, kProfMis);
                 }
+                // lmax <= mid_cap: the batch's max_hap_len bounds every window (vtx_k_locus_prep gives a wider one no tiles)
                 const int lmax = max(mid_ref, mid_alt);
                 for (int idx = lane; idx < lmax * 8; idx += 32) {
                     const int k = idx >> 3;
@@ -140,10 +213,12 @@ __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
                     midtab[idx] = pack2(r == rb ? kProfMatch : kProfMis, r == ab ? kProfMatch : kProfMis);
                 }
             }
-            // ---- row codes, forward and reversed: the 8 lanes of a unit fill their read ----
+            // ---- row codes: the 8 lanes of a unit fill their read, one byte per row ----
             const uint32_t pair = p0 + u;
             const bool active = pair < p_end;
             int m = 0;
+            uint8_t* cw = codes + u * kFoldCodeStride;
+            bool mixed;                                          // some read of the tile has a base other than ACGT
             {
                 const uint8_t* nib = nullptr;
                 if (active) {
@@ -151,17 +226,23 @@ __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
                     m = int(__ldg(a.read_len + rd));
                     nib = a.read_nib + __ldg(a.read_off + rd);
                 }
-                uint8_t* cf = codes + (2 * u) * kFoldCodeStride;
-                uint8_t* cr = cf + kFoldCodeStride;
-                for (int e = g; e < kFoldCodeStride; e += 8)
-                    if (e < M || e >= M + m) { cf[e] = 4; cr[e] = 4; }
-                for (int b = g; 2 * b < m; b += 8) {
+                bool other = false;
+                for (int b = g; 2 * b < m; b += 8) {             // forward codes 0..4 first
                     const uint32_t by = __ldg(nib + b);
-                    const uint8_t c0 = uint8_t(nib_code(by >> 4)), c1 = uint8_t(nib_code(by & 0xF));
-                    cf[M + 2 * b] = c0;
-                    cr[M + m - 1 - 2 * b] = c0;
-                    if (2 * b + 1 < m) { cf[M + 2 * b + 1] = c1; cr[M + m - 2 - 2 * b] = c1; }
+                    const uint32_t c0 = nib_code(by >> 4), c1 = nib_code(by & 0xF);
+                    cw[M + 2 * b] = uint8_t(c0);
+                    other |= c0 == 4;
+                    if (2 * b + 1 < m) { cw[M + 2 * b + 1] = uint8_t(c1); other |= c1 == 4; }
                 }
+                mixed = __any_sync(0xffffffffu, other);
+                __syncwarp();
+                for (int i = g; 2 * i < m; i += 8) {             // then row i and its mirror m - 1 - i together, in place
+                    const uint32_t x = cw[M + i], y = cw[M + m - 1 - i];
+                    cw[M + i] = uint8_t(mixed ? x << 3 | y : 4 * x + y);
+                    cw[M + m - 1 - i] = uint8_t(mixed ? y << 3 | x : 4 * y + x);
+                }
+                for (int e = g; e < kFoldCodeStride; e += 8)
+                    if (e < M || e >= M + m) cw[e] = mixed ? kFoldSentinelMixed : kFoldSentinel;
             }
             int mmax = m;
 #pragma unroll
@@ -173,63 +254,12 @@ __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
             // 0..2 of the next read, which that read wrote 150 steps earlier and nobody reads; the last read has 4 spare.
             uint2* my_bnd = bnd + u * kFoldRows;
             const uint2* row_bnd = my_bnd + 7;
-            uint32_t best;
             // =========================== main pass: forward prefix | reversed suffix ===========================
-            {
-                uint32_t hg[C1], f[C1];
+            uint32_t best = mixed ? fold_main_pass<true>(prof, cw + M - g, mmax + 7, g, one, my_bnd)
+                                  : fold_main_pass<false>(prof, cw + M - g, mmax + 7, g, one, my_bnd);
 #pragma unroll
-                for (int c = 0; c < C1; ++c) { hg[c] = kGOE2; f[c] = kNEG2; }
-                uint32_t hg_last = kGOE2, e_last = kNEG2, diag_save = kGOE2;
-                best = kBIAS2;
-                const uint8_t* cA = codes + (2 * u) * kFoldCodeStride + M - g;
-                const uint8_t* cB = cA + kFoldCodeStride;
-                const uint32_t* lane_f = profF + g * C1;
-                const uint32_t* lane_r = profR + g * C1;
-                const int steps = mmax + 7;
-#pragma unroll kFoldUnroll
-                for (int t = 0; t < steps; ++t) {
-                    uint32_t hl = __shfl_up_sync(0xffffffffu, hg_last, 1, 8);
-                    uint32_t el = __shfl_up_sync(0xffffffffu, e_last, 1, 8);
-                    if (g == 0) { hl = kGOE2; el = kNEG2; }
-                    const uint4* pa = reinterpret_cast<const uint4*>(lane_f + uint32_t(cA[t]) * RS1);
-                    const uint4* pb = reinterpret_cast<const uint4*>(lane_r + uint32_t(cB[t]) * RS1);
-                    uint32_t diag = diag_save;
-                    diag_save = hl;
-                    uint32_t e = el, eg = hl, hleft = hl;
-#pragma unroll
-                    for (int q = 0; q < C1 / 4; ++q) {
-                        const uint4 a4 = pa[q], b4 = pb[q];
-                        // {s_fwd, s_rev} = s_fwd + (s_rev << 16) as an IMAD (FMA pipe), like vtx_k_sw_split's phase 1
-#if VTX_FOLD_PRESHIFT
-                        const uint32_t sv[4] = { b4.x + a4.x, b4.y + a4.y, b4.z + a4.z, b4.w + a4.w };
-#else
-                        const uint32_t sv[4] = { b4.x * k64k + a4.x, b4.y * k64k + a4.y, b4.z * k64k + a4.z, b4.w * k64k + a4.w };
-#endif
-                        uint32_t hh[4];
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            const int c = 4 * q + k;
-                            const uint32_t fc = __viaddmax_s16x2(f[c], kGE2, hg[c]);
-                            e = __viaddmax_s16x2(e, kGE2, eg);
-                            const uint32_t h = sw_h(diag, one, sv[k], fc, e);
-                            hh[k] = h;
-                            diag = hg[c];
-                            hleft = hadd(h, one, c);
-                            eg = hleft;
-                            hg[c] = hleft;
-                            f[c] = fc;
-                        }
-                        best = __vimax3_s16x2(best, hh[0], hh[1]);
-                        best = __vimax3_s16x2(best, hh[2], hh[3]);
-                    }
-                    hg_last = hleft;
-                    e_last = e;
-                    if (g == 7) my_bnd[t] = make_uint2(hleft, e);                    // columns P-1 (fwd) / n-P (rev) of row t-7
-                }
-#pragma unroll
-                for (int o = 4; o >= 1; o >>= 1) best = __vmaxs2(best, __shfl_xor_sync(0xffffffffu, best, o));
-                best = __vmaxs2(best, __byte_perm(best, 0, 0x1032));                 // both halves: max(prefix, suffix)
-            }
+            for (int o = 4; o >= 1; o >>= 1) best = __vmaxs2(best, __shfl_xor_sync(0xffffffffu, best, o));
+            best = __vmaxs2(best, __byte_perm(best, 0, 0x1032));                     // both halves: max(prefix, suffix)
             __syncwarp();
 
             // =========================== middle: (ref, alt) over the allele columns, rows in registers ===========================
@@ -237,7 +267,8 @@ __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
                 const int lmax = max(mid_ref, mid_alt), lmin = min(mid_ref, mid_alt);
                 const uint32_t short_mask = mid_ref < mid_alt ? 0x0000FFFFu : 0xFFFF0000u;   // half whose allele ends first
                 uint32_t hg[R], e[R], rc[R];
-                const uint8_t* cf = codes + (2 * u) * kFoldCodeStride + M + R * g;
+                const uint8_t* cf = cw + M + R * g;
+                const uint32_t fwd_shift = mixed ? 3 : 2;                            // code byte -> forward code
 #pragma unroll
                 for (int c = 0; c < R; ++c) {
                     const int row = R * g + c;
@@ -245,7 +276,7 @@ __global__ void __launch_bounds__(kFoldThreads, 2) vtx_k_sw_fold(const SwArgs a)
                     if (row < mmax) b = row_bnd[row];
                     hg[c] = __byte_perm(b.x, 0, 0x1010);                             // forward half, for ref and alt
                     e[c] = __byte_perm(b.y, 0, 0x1010);
-                    rc[c] = uint32_t(cf[c]) * 4u;
+                    rc[c] = (uint32_t(cf[c]) >> fwd_shift) * 4u;                     // kFoldSentinel -> 4: matches nothing
                 }
                 // junction of the halves in `mask`: forward row r meets reversed row m - 2 - r
                 auto junction = [&](uint32_t mask) {
